@@ -83,6 +83,26 @@ class ClockSampler:
                 reasons=sorted(reasons), samples=len(sm))
 
 
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, arrays):
+  """Write what the timed path returned in its last step as <out_dir>/<name>.npy (float64 stays float64, everything
+  else is written as float32).  Above DUMP_LIMIT_BYTES in all, the same images (dim 0) of every array are kept, chosen
+  by a fixed seed, so that two builds run with the same arguments can be compared array by array."""
+  os.makedirs(out_dir, exist_ok=True)
+  arrays = {k: v.detach().cpu() for k, v in arrays.items()}
+  arrays = {k: v.double() if v.dtype == torch.float64 else v.float() for k, v in arrays.items()}
+  n = arrays[next(iter(arrays))].shape[0]
+  per_image = sum(v[0].numel() * v.element_size() for v in arrays.values())
+  keep = min(n, DUMP_LIMIT_BYTES // per_image)
+  if keep < n:
+    idx = torch.randperm(n, generator=torch.Generator().manual_seed(0))[:keep].sort().values
+    arrays = {k: v[idx] for k, v in arrays.items()}
+  for k, v in arrays.items():
+    np.save(os.path.join(out_dir, k + '.npy'), v.numpy())
+
+
 SEPARATE_GROUPNORM_DEFAULT = True   # the plan bench.py measures by default = the package default (the faster one in the same-run A/B; both are in `variants`)
 
 
@@ -140,7 +160,17 @@ def import_reference():
     m = types.ModuleType('ml_collections')
     m.ConfigDict = ConfigDict
     sys.modules['ml_collections'] = m
-  os.environ.setdefault('TORCH_EXTENSIONS_DIR', REF_EXT_DIR)      # the two JIT extensions of op/ were pre-built there
+  if 'TORCH_EXTENSIONS_DIR' not in os.environ:
+    # the two JIT extensions of op/ were pre-built in REF_EXT_DIR; torch takes a lock file in its extension directory
+    # even to load them, so they load from a temporary copy and the tree stays untouched (it may be read-only)
+    import atexit
+    import shutil
+    import tempfile
+    ext_dir = tempfile.mkdtemp(prefix='score_sde_ref_ext_')
+    atexit.register(shutil.rmtree, ext_dir, True)
+    if os.path.isdir(REF_EXT_DIR):
+      shutil.copytree(REF_EXT_DIR, ext_dir, dirs_exist_ok=True, ignore=shutil.ignore_patterns('lock'))
+    os.environ['TORCH_EXTENSIONS_DIR'] = ext_dir
   os.environ.setdefault('TORCH_CUDA_ARCH_LIST', '10.0')
   # our own package has modules of the same names (sampling, sde_lib, ...) under score_sde_pytorch_b200/, never
   # top-level, so putting the reference first on sys.path shadows nothing of ours
@@ -183,7 +213,7 @@ def reference_pc_steps(batch, steps, warmup):
       if i >= warmup:
         times.append(time.perf_counter() - t0)
   assert torch.isfinite(x_mean).all()
-  return times, 'reference'
+  return times, 'reference', dict(x=x, x_mean=x_mean)
 
 
 def port_pc_steps(batch, steps, warmup):
@@ -206,10 +236,10 @@ def port_pc_steps(batch, steps, warmup):
       t0 = time.perf_counter()
       vec_t = torch.ones(batch) * ts[i]
       x, _ = SO.langevin_step(sde, model, x, vec_t, cfg.sampling.snr, 1)
-      x, _ = SO.reverse_diffusion_step(sde, model, x, vec_t)
+      x, x_mean = SO.reverse_diffusion_step(sde, model, x, vec_t)
       if i >= warmup:
         times.append(time.perf_counter() - t0)
-  return times, 'port'
+  return times, 'port', dict(x=x, x_mean=x_mean)
 
 
 def cpu_pc_steps(batch, steps, warmup):
@@ -217,10 +247,10 @@ def cpu_pc_steps(batch, steps, warmup):
   threads = int(os.environ.get('B200_BENCH_CPU_THREADS', '0')) or len(physical_cores())
   torch.set_num_threads(threads)
   try:
-    times, kind = reference_pc_steps(batch, steps, warmup)
+    times, kind, outputs = reference_pc_steps(batch, steps, warmup)
   except (FileNotFoundError, ImportError) as err:
     print(f'bench: reference unavailable ({err}); timing the oracle port instead', file=sys.stderr)
-    times, kind = port_pc_steps(batch, steps, warmup)
+    times, kind, outputs = port_pc_steps(batch, steps, warmup)
   t_med, t_mean = float(np.median(times)), float(np.mean(times))
   spread = (max(times) - min(times)) / t_med if len(times) > 1 else 0.0
   what = ("the reference's own NCSNpp + shared_corrector_update_fn/shared_predictor_update_fn (baseline/_ref, unmodified)"
@@ -229,7 +259,7 @@ def cpu_pc_steps(batch, steps, warmup):
               sample=f'{steps} PC iterations (2 network evals each) of {what} at batch {batch} after {warmup} warm-up; '
                      f'median {t_med:.3f} s/iteration (mean {t_mean:.3f}, spread {spread:.1%}), extrapolated to '
                      f'{N_SAMPLER_STEPS} iterations; {threads} threads pinned to physical cores',
-              host_cpus=os.cpu_count(), ms_per_step=t_med * 1e3, iter_seconds=[round(t, 4) for t in times])
+              host_cpus=os.cpu_count(), ms_per_step=t_med * 1e3, iter_seconds=[round(t, 4) for t in times]), outputs
 
 
 def pinned_env():
@@ -266,9 +296,8 @@ def run_reference_arm(args):
   if os.environ.get('B200_BENCH_CPU_PINNED') != '1':
     # thread count and binding must be in the environment before libgomp starts: re-exec once
     os.execve(sys.executable, [sys.executable] + sys.argv, pinned_env())
-  batch = args.cpu_batch
-  steps = max(args.steps, 5)                 # >= 5 timed iterations: the median is the reported figure
-  r = cpu_pc_steps(batch, steps, max(args.warmup, 1))
+  batch, steps = args.cpu_batch, args.steps
+  r, outputs = cpu_pc_steps(batch, steps, max(args.warmup, 1))
   line = dict(impl='reference', metric='PC-sampler images/sec, NCSN++ CIFAR-10 1000-step VE', value=r['value'],
               unit='images/s', n_gpus=args.gpus, steps=steps, warmup=max(args.warmup, 1), ms_per_step=r['ms_per_step'],
               higher_is_better=True, scaling='weak', vs_baseline=None, dtype='f32', data='synthetic',
@@ -279,6 +308,8 @@ def run_reference_arm(args):
               e2e=dict(value=r['value'], unit='images/s', h2d_bytes_per_step=0, d2h_bytes_per_step=0),
               gpu_launches=0)
   print(json.dumps(line), flush=True)
+  if args.dump_outputs:
+    dump_outputs(args.dump_outputs, outputs)
 
 
 # ----------------------------------------------------------------------------------------------
@@ -482,6 +513,7 @@ def run_gpu_arm(args):
   clk = clocks.stop()
   ms = e0.elapsed_time(e1)
   finite = bool(torch.isfinite(x_mean).all().item())
+  outputs = dict(x=x.cpu(), x_mean=x_mean.cpu()) if args.dump_outputs and rank == 0 else None   # the e2e leg reuses these buffers
 
   # ---- end to end through the public plan API with host buffers, copies inside the timed region ----
   e2e_steps = args.steps
@@ -645,6 +677,8 @@ def run_gpu_arm(args):
     if parity is not None:
       line['parity'] = parity
     print(json.dumps(line), flush=True)
+    if outputs is not None:
+      dump_outputs(args.dump_outputs, outputs)
   if world > 1:
     dist.destroy_process_group()
 
@@ -702,6 +736,7 @@ def run_secondary_workload(args):
                             step='one right-hand side = one network evaluation + Dormand-Prince stage arithmetic in float64 on the device',
                             weights='random init, init_scale=1, torch.manual_seed(0)'),
                 clocks=clocks, finite=bool(torch.isfinite(s).all()), gpu_launches=int(model.launches_per_forward()) * int(nfe))
+    outputs = dict(samples=s)
   else:
     plan = native.match_pc_plan(sde=sde, model=model, predictor=W['pred'], corrector=W['corr'], shape=shape, snr=W['snr'], n_steps=1,
                                 probability_flow=False, continuous=True, eps=W['eps'], device=dev)
@@ -717,7 +752,10 @@ def run_secondary_workload(args):
                 config=dict(workload=W['desc'], batch_per_gpu=B, sampler_steps=N, score_evaluations_per_step=W['evals'],
                             parameters=sum(p.numel() for p in model.parameters()), weights='random init, init_scale=1, torch.manual_seed(0)'),
                 clocks=clocks, finite=bool(torch.isfinite(plan._xm).all()), gpu_launches=int(plan.launches_per_step()) * args.steps)
+    outputs = dict(x=plan._x, x_mean=plan._xm)     # what plan.run(..., clone=False) handed back in the last timed call
   print(json.dumps(line), flush=True)
+  if args.dump_outputs:
+    dump_outputs(args.dump_outputs, outputs)
 
 
 def main():
@@ -742,6 +780,8 @@ def main():
                   help='PC iterations of the in-run parity check against the strict-fp32 GPU oracle at the full batch (0 = skip)')
   ap.add_argument('--scaling', default='weak', choices=['weak', 'strong'],
                   help="'weak' (default, headline): --batch images per GPU; 'strong': --batch images in total, cut over the ranks")
+  ap.add_argument('--dump-outputs', metavar='DIR',
+                  help='after the timed steps, write what the timed path returned in its last step as DIR/<name>.npy')
   ap.add_argument('--workload', default='cifar10_ve',
                   choices=['cifar10_ve', 'cifar10_ddpmpp_vp', 'celebahq_256_ve', 'ffhq_1024_ve', 'celebahq_256_ddpmpp_subvp_ode'],
                   help="'cifar10_ve' (default) is the headline line; the others print one line for a secondary configuration (1 GPU)")

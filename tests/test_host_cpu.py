@@ -289,7 +289,7 @@ def test_product_model_has_no_cpu_path():
     seeded_model(cfg)
 
 
-def test_bench_reference_arm_prints_the_contract_line():
+def test_bench_reference_arm_prints_the_contract_line(tmp_path):
   """`bench.py --impl reference` (the CPU arm the driver runs beside the GPU arm): one JSON line with the same
   metric/unit/config keys, `impl: reference`, a cpu_baseline describing the run and a zero-copy e2e block."""
   import json
@@ -298,8 +298,8 @@ def test_bench_reference_arm_prints_the_contract_line():
   import sys
   root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
   env = dict(os.environ, OMP_NUM_THREADS='1')      # what torchrun exports to every rank
-  out = subprocess.run([sys.executable, os.path.join(root, 'bench.py'), '--impl', 'reference', '--steps', '1', '--warmup', '0',
-                        '--cpu-batch', '1'], capture_output=True, text=True, timeout=900, env=env, cwd=root)
+  out = subprocess.run([sys.executable, os.path.join(root, 'bench.py'), '--impl', 'reference', '--steps', '5', '--warmup', '0',
+                        '--cpu-batch', '1', '--dump-outputs', str(tmp_path / 'out')], capture_output=True, text=True, timeout=900, env=env, cwd=root)
   assert out.returncode == 0, out.stderr[-2000:]
   line = json.loads(out.stdout.strip().splitlines()[-1])
   assert line['impl'] == 'reference' and line['unit'] == 'images/s' and line['higher_is_better'] is True
@@ -308,10 +308,33 @@ def test_bench_reference_arm_prints_the_contract_line():
   # the UNMODIFIED reference from baseline/_ref (tools/install_ref.sh) when it is installed, else the oracle port
   want = 'reference' if os.path.isdir(os.path.join(root, 'baseline', '_ref', 'models')) else 'port'
   assert cb['kind'] == want and cb['value'] == line['value'] and cb['cores'] >= 1 and 'PC iterations' in cb['sample']
-  assert line['steps'] >= 5 and len(cb['iter_seconds']) == line['steps']      # the median of >= 5 iterations is reported
+  assert line['steps'] == 5 and len(cb['iter_seconds']) == 5      # --steps sets the timed iterations; their median is reported
   assert line['e2e'] == {'value': line['value'], 'unit': 'images/s', 'h2d_bytes_per_step': 0, 'd2h_bytes_per_step': 0}
   if (os.cpu_count() or 1) >= 4:
     assert cb['cores'] > 1        # OMP_NUM_THREADS=1 from the launcher must not reduce the arm to one core
+  import numpy as np
+  for name in ('x', 'x_mean'):    # the state the last timed PC iteration returned
+    a = np.load(tmp_path / 'out' / f'{name}.npy')
+    assert a.dtype == np.float32 and a.shape == (1, 3, 32, 32) and np.isfinite(a).all()
+
+
+def test_bench_dump_outputs_keeps_a_fixed_sample_under_the_size_limit(tmp_path, monkeypatch):
+  import os
+  import sys
+  import numpy as np
+  sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
+  import bench
+  x = torch.arange(10 * 6, dtype=torch.float32).reshape(10, 2, 3)
+  xm = x.double() * 2
+  bench.dump_outputs(str(tmp_path / 'all'), dict(x=x, x_mean=xm))
+  assert np.array_equal(np.load(tmp_path / 'all' / 'x.npy'), x.numpy())
+  assert np.load(tmp_path / 'all' / 'x_mean.npy').dtype == np.float64
+  monkeypatch.setattr(bench, 'DUMP_LIMIT_BYTES', 4 * (6 * 4 + 6 * 8))     # room for four images of both arrays
+  for d in ('a', 'b'):
+    bench.dump_outputs(str(tmp_path / d), dict(x=x, x_mean=xm))
+  a, am = np.load(tmp_path / 'a' / 'x.npy'), np.load(tmp_path / 'a' / 'x_mean.npy')
+  assert a.shape == (4, 2, 3) and np.array_equal(am, a.astype(np.float64) * 2)   # the same images of every array
+  assert np.array_equal(a, np.load(tmp_path / 'b' / 'x.npy'))                   # the same images on every run
 
 
 def test_ema_matches_reference_update_rule_and_notifies_the_engine_module(tmp_path):

@@ -26,10 +26,11 @@ def test_ncsnpp_oracle_matches_reference(name):
   taps = {}
   with torch.no_grad():
     y = NO.ncsnpp_forward(sd, cfg, torch.from_numpy(g['x']), torch.from_numpy(g['sigma']), taps=taps)
+  stride = int(g.get('tap_stride', 1))       # larger fixtures keep every stride-th element of each image's activation
   for i, v in sorted(taps.items()):
     key = f'tap{i}'
     if key in g:
-      assert rel_l2(v, torch.from_numpy(g[key])) < 2e-6, f'module {i} diverges from the reference'
+      assert rel_l2(v.reshape(len(v), -1)[:, ::stride], torch.from_numpy(g[key])) < 2e-6, f'module {i} diverges from the reference'
   assert rel_l2(y, torch.from_numpy(g['y'])) < 2e-6
 
 

@@ -43,9 +43,10 @@ def main():
       ref_model(x, sigma)
       for h in hooks:
         h.remove()
-    rec = dict(x=x.numpy(), sigma=sigma.numpy(), y=y.numpy())
+    # every third element of each image's activation keeps the fixture under 1 MB (tests/test_oracle_golden.py reads tap_stride)
+    rec = dict(x=x.numpy(), sigma=sigma.numpy(), y=y.numpy(), tap_stride=np.array(3))
     for i, v in taps.items():
-      rec[f'tap{i}'] = v.numpy()
+      rec[f'tap{i}'] = np.ascontiguousarray(v.reshape(B, -1)[:, ::3].numpy())
     np.savez_compressed(os.path.join(MG.OUT, f'ncsnpp_{name}.npz'), **rec)
     print(name, 'forward done', float(y.abs().mean()), 'modules', len(ref_model.all_modules))
   # full-size members: key / shape layout only (the 1024x1024 forward is a GPU job)
